@@ -6,6 +6,7 @@ synthetic 550x550 frames, yolact_base (ResNet101-FPN), batch 8 per GPU (BASELINE
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
 
 One step = one batch through the whole path.  Prints ONE JSON line (rank 0).  See DESIGN.md
 "Measurement" for what each key means; in short:
@@ -64,7 +65,12 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=16, help="images in the cpu_baseline sample")
     ap.add_argument("--top-k", dest="top_k", type=int, default=5,
                     help="detections per image copied to the host in the e2e loop (eval.py --top_k default: 5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of `value` returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -224,6 +230,27 @@ def time_cpu(cfg, sd, size, batch, steps, warmup, seed=8000):
     return batch * steps / dt, dt / steps, nd / float(max(1, batch * steps))
 
 
+MASK_SAMPLES = 1 << 21   # fp32 mask values kept by dump_outputs: 8 MB, plus 16 MB of float64 indices
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes one step's outputs of the `value` path as out_dir/<name>.npy, so that two builds run with the same
+    arguments (hence the same seeded inputs and weights) can be compared array by array.  Integer arrays are stored
+    as float64, which holds them exactly.  The fp32 masks [B, M, h, w] are about 1 GB at the default workload, so
+    only a fixed, seeded sample of their elements is written, with its flat indices."""
+    import numpy as np
+    import torch
+    box, coef, cls, score, count, (masks, boxes_px) = outputs
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randint(0, masks.numel(), (min(MASK_SAMPLES, masks.numel()),), generator=g).sort().values
+    arrays = {"box": box, "coef": coef, "class": cls, "score": score, "count": count, "box_px": boxes_px,
+              "masks_sample": masks.reshape(-1)[idx.to(masks.device)], "masks_sample_index": idx}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def workload_string(cfg, size, B):
     return "%s @%d, batch %d/GPU, synthetic frames, random-init deterministic weights (100 detections/image)" % (
         cfg.name, size, B)
@@ -372,11 +399,18 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms = timed(lambda i: step_device(net, i, "f32", masks_f32), args.steps, max(3, args.warmup))
+    last = {}
+
+    def step_value(i):
+        last["out"] = step_device(net, i, "f32", masks_f32)
+    ms = timed(step_value, args.steps, max(3, args.warmup))
     clocks = sampler.stop() if rank == 0 else None
     # kernels launched inside the TIMED region only (the counter also saw the warm-up steps of `timed`)
     launches = (net.launch_count() + output_utils.launch_count() - l0) * args.steps // (args.steps + max(3, args.warmup))
     fps = world * B * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["out"])   # timed() has synchronised: the last step is complete
+    last.clear()
     hold[0] = hold[1] = None
 
     # ---- e2e (headline): the reference-facing API with HOST frames, eval.py's --benchmark protocol --------------------

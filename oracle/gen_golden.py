@@ -1,6 +1,6 @@
-"""Generates tests/golden/*.npz by running the REAL reference (/root/reference) on this container's CPU.
+"""Generates tests/golden/* by running the REAL reference (an upstream YOLACT checkout) on the CPU.
 
-Run here (the GPU box has no /root/reference):   python oracle/gen_golden.py
+    python oracle/gen_golden.py [keys|units|eval|cfgs|full|nets ...]   # reference located by oracle/build_ref.py
 The committed .npz files are what pins oracle/yolact_oracle.py and the CUDA path to the reference.
 
 Shims (never edits to the reference; SURVEY.md section 8c): stub pycocotools / matplotlib in
@@ -18,7 +18,8 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+from oracle.build_ref import reference_root  # noqa: E402
+REF = reference_root() or ""
 OUT = os.path.join(ROOT, "tests", "golden")
 
 
@@ -469,7 +470,42 @@ def gen_state_keys():
         json.dump(out, f)
 
 
+def gen_reference_cfgs():
+    """Every published config as plain JSON: exactly the fields yolact_b200.config.from_reference_cfg reads, so that
+    the tests (tests/helpers.py load_reference_cfgs) can rebuild duck-typed cfg objects without the reference tree."""
+    import json
+    from data import config as rc
+    switches = ("use_prediction_module", "use_yolo_regressors", "use_mask_scoring", "use_instance_coeff", "use_focal_loss",
+                "use_objectness_score", "mask_proto_use_grid", "mask_proto_coeff_gate", "mask_proto_prototypes_as_features",
+                "mask_proto_split_prototypes_by_head", "mask_proto_bias", "share_prediction_module", "use_maskiou",
+                "rescore_mask", "rescore_bbox", "eval_mask_branch", "mask_proto_debug", "preserve_aspect_ratio")
+    scalars = ("name", "max_size", "num_classes", "mask_dim", "nms_top_k", "nms_conf_thresh", "nms_thresh",
+               "max_num_detections")
+    out = {}
+    for name in ("yolact_base_config", "yolact_resnet50_config", "yolact_im700_config", "yolact_darknet53_config",
+                 "yolact_plus_base_config", "yolact_plus_resnet50_config"):
+        c = getattr(rc, name)
+        b = c.backbone
+        d = {k: getattr(c, k) for k in scalars + switches if hasattr(c, k)}
+        d["fpn"] = {"num_features": c.fpn.num_features}
+        d["backbone"] = {
+            "type": b.type.__name__, "args": [list(a) if isinstance(a, (list, tuple)) else a for a in b.args],
+            "selected_layers": list(b.selected_layers), "pred_scales": [[float(v) for v in s] for s in b.pred_scales],
+            "pred_aspect_ratios": [[list(r) for r in a] for a in b.pred_aspect_ratios],
+            "use_square_anchors": b.use_square_anchors,
+            "transform": {k: getattr(b.transform, k) for k in ("channel_order", "normalize", "subtract_means", "to_float")
+                          if hasattr(b.transform, k)}}
+        out[name] = d
+        print("reference cfg", name, d["backbone"]["type"], d["backbone"]["args"])
+    os.makedirs(OUT, exist_ok=True)
+    with open(os.path.join(OUT, "reference_cfgs.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 if __name__ == "__main__":
+    if not os.path.isfile(os.path.join(REF, "eval.py")):
+        raise SystemExit("no reference tree: set YOLACT_REFERENCE to the root of an upstream YOLACT checkout")
     install_shims()
     torch.set_num_threads(8)
     which = sys.argv[1:] or ["units", "nets"]
@@ -481,6 +517,8 @@ if __name__ == "__main__":
         gen_dcn_unit()
     if "units" in which or "eval" in which:
         gen_eval_unit()
+    if "units" in which or "cfgs" in which:
+        gen_reference_cfgs()
     if "full" in which:
         for tag, name, size, post in FULL_CASES:
             gen_fullsize_case(tag, name, size, post)

@@ -42,7 +42,9 @@ def _worker(rank, world, port, q):
     mine = _fake(rank, e - s)
     out = gather_detections(*mine, per_rank_batch=3)
     if rank == 0:
-        q.put([t.clone() for t in out])
+        # numpy arrays travel by value: a tensor's storage is shared through a socket of this process, which may
+        # already have exited when the parent unpickles it
+        q.put([t.numpy().copy() for t in out])
     dist.barrier()
     dist.destroy_process_group()
 
@@ -56,7 +58,7 @@ def test_gather_detections_world2_gloo():
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    out = q.get(timeout=120)
+    out = [torch.from_numpy(a) for a in q.get(timeout=120)]
     for p in procs:
         p.join(timeout=120)
         assert p.exitcode == 0
